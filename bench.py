@@ -17,6 +17,10 @@ the same graph (tests/golden/golden_full_<nv>_p<N>.json: iteration count, every 
 hash) triple, final assignment hash); a mismatch aborts the benchmark with a non-zero exit code.
 Timing: CUDA events on the library's stream (max over ranks) for `value`; inputs (3 GB/GPU) exceed L2 so
 no explicit flush is needed between steps.
+--dump-outputs DIR: after the timed steps, what the last timed `value` step returned to its caller is written as
+DIR/<name>.npy (float64): modularity, iterations, and the final community of a fixed, seeded sample of at most 2^21
+vertices (community_vertices.npy holds their global ids).  The graph is a function of the arguments, so two builds
+run with the same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -32,9 +36,12 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 NV_PER_GPU = 16777216
 METRIC = "louvain_phase_edges_per_sec"
+DUMP_SAMPLE = 1 << 21               # --dump-outputs: vertices whose community is written (2 x 16 MB of float64)
+DUMP_SEED = 20240601
 
 
 def load_peaks():
@@ -161,7 +168,8 @@ def reference_runs(nv_total, N, max_timed, budget_s, verbose=False, fallback_nv=
     """Time oracle/_ref/miniVite_ref -- the unmodified reference -- on the benchmark graph itself (N strips, read with
     -f), in its genuine MPI+OpenMP mode: N ranks x (cores/N) OpenMP threads (N=1: one rank x all cores).  One warm-up
     run, then up to `max_timed` timed runs while the time budget lasts; if a single run does not fit the budget the
-    run that was made is the sample.  Only if the reference binary is missing does the C restatement stand in."""
+    run that was made is the sample.  Only if the reference binary is missing does the C restatement stand in: on the
+    benchmark graph itself up to `fallback_nv` vertices, on the 1-strip RGG of `fallback_nv` vertices above that."""
     from minivite_b200 import hostgraph as hg
     from oracle import oracle as O
     cores, cores_detail = host_cores()
@@ -170,15 +178,18 @@ def reference_runs(nv_total, N, max_timed, budget_s, verbose=False, fallback_nv=
     ss = hg.generate_rgg(nv_total, N)
     ne = sum(s.lne for s in ss.shards)
     if not O.have_reference():
-        ss.close()
-        ss = hg.generate_rgg(fallback_nv, 1)
-        sh = ss.shards[0]
+        same = nv_total <= fallback_nv
+        if not same:
+            ss.close()
+            ss = hg.generate_rgg(fallback_nv, 1)
         t = time.time()
-        r = O.louvain(sh.parts, [sh.rowptr], [sh.edges])
+        r = O.louvain(ss.shards[0].parts, [s.rowptr for s in ss.shards], [s.edges for s in ss.shards])
         t = time.time() - t
-        return {"value": sh.lne * r["iters"] / t, "ms_per_step": t * 1e3, "cores": 1, "kind": "port", "ne": ne,
-                "unit": "edges/s", "same_graph": False, "runs_timed": 1, "cores_detail": cores_detail,
-                "sample": f"oracle/_ref absent: C restatement, 1 thread, RGG n={fallback_nv} full Louvain phase"}
+        return {"value": sum(s.lne for s in ss.shards) * r["iters"] / t, "ms_per_step": t * 1e3, "cores": 1,
+                "kind": "port", "ne": ne, "unit": "edges/s", "same_graph": same, "runs_timed": 1,
+                "cores_detail": cores_detail,
+                "sample": f"oracle/_ref absent: C restatement, 1 thread, RGG n={nv_total if same else fallback_nv} "
+                          f"({N if same else 1} strip(s)) full Louvain phase"}
     tmp = scratch_dir(16 * ne + 8 * nv_total)
     path = os.path.join(tmp, "g.bin")
     ss.write(path)
@@ -230,7 +241,11 @@ def main():
                          "the copy engine additionally takes raw chunks from the far end whenever no narrowed chunk is ready")
     ap.add_argument("--ref-budget-s", type=float, default=420.0, help="wall-clock budget of the reference arm's runs")
     ap.add_argument("--verbose", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (modularity, iterations, sampled communities) as DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -396,6 +411,22 @@ def main():
     info = ctx.shard_info()
     if not args.no_parity:
         assert iters == iters_p and mod == mod_p, "timed runs disagree with the parity run"
+    if args.dump_outputs:
+        # the last timed step's assignment at a fixed, seeded sample of global vertex ids; each rank fills the entries
+        # it owns and a sum over ranks (exact: every entry has one non-zero contribution) assembles the sample
+        idx = (np.sort(np.random.default_rng(DUMP_SEED).choice(nv_total, DUMP_SAMPLE, replace=False))
+               if nv_total > DUMP_SAMPLE else np.arange(nv_total, dtype=np.int64))
+        comm = ctx.communities(out=torch.empty(sh.lnv, dtype=torch.int64).pin_memory().numpy())
+        own = (idx >= parts[rank]) & (idx < parts[rank + 1])
+        sampled = np.zeros(len(idx), np.float64)
+        sampled[own] = comm[idx[own] - parts[rank]]
+        if world > 1:
+            buf = torch.from_numpy(sampled).cuda()
+            dist.all_reduce(buf)
+            sampled = buf.cpu().numpy()
+        outputs = {"modularity": np.array([mod], np.float64), "iterations": np.array([iters], np.float64),
+                   "communities": sampled, "community_vertices": idx.astype(np.float64)}
+        del comm
 
     # ---- e2e: host arrays -> H2D -> Louvain -> assignment D2H, through the public API
     cu_threads = args.compact_upload if args.compact_upload >= 0 else max(1, min(32, cores // max(world, 1)))
@@ -429,6 +460,10 @@ def main():
             dist.destroy_process_group()
         return 0
 
+    if args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     peak, peak_src = load_peaks()
     lnv, lne = sh.lnv, sh.lne
     b_alg = 24.0 * lne + 56.0 * lnv            # SURVEY.md 8(d): reference element sizes, per scan launch per GPU

@@ -1,8 +1,11 @@
-"""bench.py contract (CPU part): the reference arm prints exactly ONE JSON line on stdout with the agreed keys."""
+"""bench.py contract: the reference arm prints exactly ONE JSON line on stdout with the agreed keys (CPU), and
+--dump-outputs writes what the timed path returned (GPU)."""
 import json
 import os
 import subprocess
 import sys
+
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -46,3 +49,26 @@ def test_reference_arm_other_ranks_exit_quietly():
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1",
                         "--warmup", "1"], capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert p.returncode == 0 and p.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_result(tmp_path, golden):
+    """At 16384 vertices the dump is the whole assignment: the graph of `miniVite -n 16384`, so the reference's
+    golden (rgg_n16384_p1) pins iterations, modularity and the final assignment hash."""
+    import numpy as np
+    from oracle import oracle as O
+    out = tmp_path / "out"
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "0", "--nv-per-gpu",
+                        "16384", "--no-cpu-baseline", "--dump-outputs", str(out)], capture_output=True, text=True,
+                       timeout=600, cwd=ROOT)
+    assert p.returncode == 0, p.stderr[-2000:]
+    d = json.loads(p.stdout)
+    assert d["steps"] == 2
+    files = {f.name: np.load(f) for f in out.iterdir()}
+    assert set(files) == {"modularity.npy", "iterations.npy", "communities.npy", "community_vertices.npy"}
+    assert all(a.dtype == np.float64 for a in files.values())
+    case = golden["rgg_n16384_p1"]
+    assert files["iterations.npy"][0] == case["iters"] == d["result"]["iterations"]
+    assert files["modularity.npy"][0] == float(case["modularity"]) == d["result"]["modularity"]
+    assert np.array_equal(files["community_vertices.npy"], np.arange(16384))
+    assert "%016x" % O.comm_hash(0, files["communities.npy"].astype(np.int64)) == case["final_chash"]

@@ -15,7 +15,7 @@ pytestmark = pytest.mark.gpu
 def _run(args, nranks=1):
     from oracle import oracle as O
     if not os.path.exists(O.REF_GPU_BIN):
-        pytest.skip("oracle/_ref/miniVite_ref_gpu not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/miniVite_ref_gpu not built (needs the reference's sources at build time)")
     return O.run_reference(args, nranks=nranks, threads=2, trace=True, binary=O.REF_GPU_BIN, timeout=600)
 
 
